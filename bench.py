@@ -2,7 +2,7 @@
 """
 bench.py — BASELINE.json metric: corpus GB/s and merges/s through the train() merge loop.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--size-mib M]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--size-mib M] [--dump-outputs DIR]
 
 A "step" is one merge iteration (get_stats -> arg-max with the reference tie-break -> merge) over
 the whole resident token stream.  Workload at N=1: BASELINE.json configs[2], RegexTokenizer.train
@@ -402,7 +402,7 @@ def run_reference(args):
     oracle.build()
     cores = min(host_cores(), 64)
     shard = 16 << 20
-    steps = max(1, min(args.steps, 8))
+    steps = args.steps
     warm = min(args.warmup, 1)
     t0 = time.perf_counter()
     solo = _ref_worker((args.seed, 0, shard, steps, warm))        # one replica alone: the per-core rate
@@ -558,6 +558,25 @@ def oracle_train_unique(chunks, weights, merges):
 def merges_sha(pairs):
     import hashlib
     return hashlib.sha256(np.ascontiguousarray(pairs, dtype=np.int32).tobytes()).hexdigest()[:16]
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, **arrays):
+    """--dump-outputs: what the timed train() call returned, one float64 `<name>.npy` per array (exact: ids are int32 and
+    counts stay below 2**53), so that two builds run with the same arguments can be compared output for output.  All
+    arrays have one row per merge; past DUMP_BYTES a fixed, seeded sample of rows is kept and its indices go to rows.npy."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = 8 + sum(a[:1].nbytes for a in arrays.values())
+    if n * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // row_bytes, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 def strong_host_bytes(args):
@@ -978,6 +997,8 @@ def run_sharded(args, rank, world, local):
     merge_all = [torch.zeros_like(merge_ms) for _ in range(world)]
     dist.all_gather(merge_all, merge_ms)
     line = None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, merges=pairs[W:W + K], counts=counts[W:W + K])
     if rank == 0:
         t = float(t_loop.item())
         peak, peak_src = measured_peak()
@@ -1130,6 +1151,8 @@ def run_ours(args):
     tm = eng.timing()
     assert done == K
     assert np.array_equal(pairs, pairs_e2e[W:W + K]), "timed run and e2e run disagree"
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, merges=pairs, counts=counts)
     t_loop = tm["loop_ms"] / 1e3          # CUDA events on the library's stream, around the K iterations
     value = size * K / t_loop / 1e9
     n_in, n_out = tm["tokens_in"], tm["tokens_out"]
@@ -1293,7 +1316,14 @@ def main():
     ap.add_argument("--no-p2p-trial", action="store_true", help="N>1: skip the trial of the NVLink peer-memory exchange kernels")
     ap.add_argument("--no-filter-leg", action="store_true", help="skip the full_run_filtered leg (N=1)")
     ap.add_argument("--extras", action="store_true", help="side measurements (cfg2 wall time, encode throughput)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what they returned to DIR as float64 .npy files: merges.npy (the K merged "
+                         "pairs, [K, 2]) and counts.npy (their occurrence counts, [K])")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.extras or args.impl != "ours"):
+        ap.error("--dump-outputs writes the outputs of the timed merge loop of --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.extras:

@@ -1,13 +1,16 @@
 #!/usr/bin/env python3
 """TEST INFRASTRUCTURE (BPE_LIB_PATH = the emulator build): RegexTokenizer.encode(text, allowed_special=...) with the
 special tokens found, the parts split and everything encoded on the device (k_special.cuh, split_logic.h WITH_B,
-k_encode2.cuh) against the UNMODIFIED reference class (oracle/_ref/minbpe, vendored by oracle/make_ref.py) on random
-texts: specials that are prefixes of one another, adjacent and overlapping occurrences, specials at either end of the
-text, white space / letters / digits / apostrophes on both sides (the split of a part must behave as on a text of its own),
-both split patterns, subsets as `allowed_special`, several pieces per call.
+k_encode2.cuh) against the ids the UNMODIFIED reference class returned for the same random texts
+(tests/golden/golden_fuzz_special.json, written by tests/golden/make_golden_ref_checks.py): specials that are prefixes of
+one another, adjacent and overlapping occurrences, specials at either end of the text, white space / letters / digits /
+apostrophes on both sides (the split of a part must behave as on a text of its own), both split patterns, subsets as
+`allowed_special`, several pieces per call.
 
-    BPE_LIB_PATH=tests/emu/_build/libb200bpe_emu.so python tests/emu/emu_fuzz_special.py [rounds] [seed]
+    BPE_LIB_PATH=tests/emu/_build/libb200bpe_emu.so python tests/emu/emu_fuzz_special.py
 """
+import hashlib
+import json
 import os
 import sys
 
@@ -15,59 +18,31 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
-from oracle import make_ref  # noqa: E402
 from minbpe_b200 import RegexTokenizer  # noqa: E402
 from minbpe_b200 import engine as E  # noqa: E402
 from minbpe_b200.tokenizer import GPT2_SPLIT_PATTERN, GPT4_SPLIT_PATTERN  # noqa: E402
 
-POOL = ["<|endoftext|>", "<|end|>", "<|endof", "<|a|>", "<|a|><|b|>", "<|b|>", "<s>", "</s>", "<s", "[SEP]", "[S", " <pad>", "<|é|>", "'s<", "12", "\n\n<|x|>"]
-FILL = list("abcde  é1!'\n\t") + ["日", " the", "'ll", "  ", "\r\n", "42"]
+
+def ids_sha(ids):
+    return hashlib.sha256(np.asarray(ids, dtype="<i4").tobytes()).hexdigest()
 
 
-def random_case(rng):
-    k = int(rng.integers(1, 6))
-    toks = [str(x) for x in rng.choice(POOL, size=k, replace=False)]
-    special = {t: 1000 + i for i, t in enumerate(toks)}
-    parts = []
-    for _ in range(int(rng.integers(1, 60))):
-        r = rng.random()
-        if r < 0.35:
-            parts.append(str(rng.choice(toks)))
-        elif r < 0.45:
-            t = str(rng.choice(toks))
-            parts.append(t[: int(rng.integers(1, len(t) + 1))])          # a truncated special: must stay ordinary text
-        else:
-            parts.append("".join(str(x) for x in rng.choice(FILL, size=int(rng.integers(1, 12)))))
-    return special, "".join(parts)
-
-
-def main(rounds, seed):
-    ref = make_ref.load()
-    if ref is None:
-        print("emu fuzz special: oracle/_ref is not vendored here (run oracle/make_ref.py where /root/reference exists)")
-        return 2
-    rng = np.random.default_rng(seed)
-    train_text = open(os.path.join(ROOT, "tests", "golden", "taylorswift.txt"), encoding="utf-8").read()[:60000]
+def main():
+    with open(os.path.join(ROOT, "tests", "golden", "golden_fuzz_special.json"), encoding="utf-8") as f:
+        g = json.load(f)
     toks = {}
-    for pat in (GPT4_SPLIT_PATTERN, GPT2_SPLIT_PATTERN):
-        r = ref.RegexTokenizer(pat)
-        r.train(train_text[:20000], 256 + 120)
+    for name, pat in (("gpt4", GPT4_SPLIT_PATTERN), ("gpt2", GPT2_SPLIT_PATTERN)):
         o = RegexTokenizer(pat)
-        o.merges, o.vocab = dict(r.merges), dict(r.vocab)
+        o.merges = {(a, b): 256 + i for i, (a, b) in enumerate(g["merges"][name])}   # the reference's trained merges
+        o.vocab = o._build_vocab()
         o.DEVICE_SPLIT_MIN_BYTES = 0          # every text takes the device path, however short
-        toks[pat] = (r, o)
+        toks[name] = o
     n_dev = 0
-    for it in range(rounds):
-        special, text = random_case(rng)
-        if rng.random() < 0.2:
-            text = text + " " + train_text[: int(rng.integers(100, 5000))] + text
-        pat = GPT4_SPLIT_PATTERN if rng.random() < 0.6 else GPT2_SPLIT_PATTERN
-        r, o = toks[pat]
-        r.register_special_tokens(special)
-        o.register_special_tokens(special)
-        allowed = "all" if rng.random() < 0.7 else set(list(special)[: int(rng.integers(0, len(special) + 1))])
-        piece = int(rng.choice([0, 0, 0, 4096]))
-        o.engine.set_option(E.OPT_SPLIT_PIECE, piece)
+    for it, c in enumerate(g["cases"]):
+        o, text = toks[c["pattern"]], c["text"]
+        o.register_special_tokens(c["special"])
+        allowed = c["allowed"] if c["allowed"] == "all" else set(c["allowed"])
+        o.engine.set_option(E.OPT_SPLIT_PIECE, c["piece"])
         try:
             try:
                 got = o.encode(text, allowed_special=allowed)
@@ -76,13 +51,12 @@ def main(rounds, seed):
                 continue
         finally:
             o.engine.set_option(E.OPT_SPLIT_PIECE, 0)
-        want = r.encode(text, allowed_special=allowed)
-        assert got == want, (it, pat == GPT4_SPLIT_PATTERN, special, allowed, text)
-        assert o.decode(got) == r.decode(want)
+        assert (len(got), ids_sha(got)) == (c["n_ids"], c["ids_sha256"]), (it, c["pattern"], c["special"], c["allowed"], text)
+        assert o.decode(got) == text
         n_dev += 1
-    print(f"emu fuzz special ok: {n_dev} of {rounds} rounds compared with the reference class")
+    print(f"emu fuzz special ok: {n_dev} of {len(g['cases'])} rounds compared with the reference class")
     return 0
 
 
 if __name__ == "__main__":
-    sys.exit(main(int(sys.argv[1]) if len(sys.argv) > 1 else 200, int(sys.argv[2]) if len(sys.argv) > 2 else 1))
+    sys.exit(main())

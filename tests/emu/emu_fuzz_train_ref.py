@@ -1,11 +1,14 @@
 #!/usr/bin/env python3
 """TEST INFRASTRUCTURE (BPE_LIB_PATH = the emulator build): BasicTokenizer / RegexTokenizer .train() of the product classes
-(kernels on the emulator) against the UNMODIFIED reference classes (oracle/_ref/minbpe) on random small texts — tie-heavy
-alphabets, runs of one character (the (a,a) path), texts that run out of pairs (both must raise ValueError and leave the
-tokenizer untrained), both split patterns; merges, vocab, the ids of encode() and the saved .model bytes must be identical.
+(kernels on the emulator) against what the UNMODIFIED reference classes did on the same random small texts
+(tests/golden/golden_fuzz_train.json, written by tests/golden/make_golden_ref_checks.py) — tie-heavy alphabets, runs of one
+character (the (a,a) path), texts that run out of pairs (both must raise ValueError and leave the tokenizer untrained),
+both split patterns; merges, vocab, the ids of encode() and the saved .model / .vocab bytes must be identical.
 
-    BPE_LIB_PATH=tests/emu/_build/libb200bpe_emu.so python tests/emu/emu_fuzz_train_ref.py [rounds] [seed]
+    BPE_LIB_PATH=tests/emu/_build/libb200bpe_emu.so python tests/emu/emu_fuzz_train_ref.py
 """
+import hashlib
+import json
 import os
 import sys
 import tempfile
@@ -14,66 +17,50 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
-from oracle import make_ref  # noqa: E402
 import minbpe_b200 as ours  # noqa: E402
 from minbpe_b200.tokenizer import GPT2_SPLIT_PATTERN, GPT4_SPLIT_PATTERN  # noqa: E402
 
 
-def random_text(rng):
-    kind = rng.random()
-    if kind < 0.3:
-        alpha = list("ab")                                   # ties everywhere, long runs
-    elif kind < 0.6:
-        alpha = list("abc de'1\n")
-    else:
-        alpha = list("the quick brown fox é日 12 's 'll\t") + ["aaaa", "  ", "zzzzzz"]
-    n = int(rng.choice([1, 2, 3, 5, 12, 40, 200, 1500]))
-    return "".join(str(x) for x in rng.choice(alpha, size=n))
+def sha(b):
+    return hashlib.sha256(b).hexdigest()
 
 
-def main(rounds, seed):
-    ref = make_ref.load()
-    if ref is None:
-        print("emu fuzz train: oracle/_ref is not vendored here")
-        return 2
-    rng = np.random.default_rng(seed)
+def main():
+    with open(os.path.join(ROOT, "tests", "golden", "golden_fuzz_train.json"), encoding="utf-8") as f:
+        cases = json.load(f)["cases"]
     done = raised = 0
     tmp = tempfile.mkdtemp()
-    for it in range(rounds):
-        text = random_text(rng)
-        vocab = 256 + int(rng.choice([0, 1, 2, 5, 20, 60]))
-        which = int(rng.integers(0, 3))
-        if which == 0:
-            r, o = ref.BasicTokenizer(), ours.BasicTokenizer()
+    for it, c in enumerate(cases):
+        text, vocab, which = c["text"], c["vocab_size"], c["tokenizer"]
+        if which == "basic":
+            o = ours.BasicTokenizer()
         else:
-            pat = GPT4_SPLIT_PATTERN if which == 1 else GPT2_SPLIT_PATTERN
-            r, o = ref.RegexTokenizer(pat), ours.RegexTokenizer(pat)
-        err_r = err_o = None
-        try:
-            r.train(text, vocab)
-        except ValueError as ex:
-            err_r = ex
+            o = ours.RegexTokenizer(GPT4_SPLIT_PATTERN if which == "gpt4" else GPT2_SPLIT_PATTERN)
+        err = None
         try:
             o.train(text, vocab)
         except ValueError as ex:
-            err_o = ex
-        assert (err_r is None) == (err_o is None), (it, which, vocab, text, err_r, err_o)
-        if err_r is not None:
+            err = ex
+        assert (err is not None) == ("raises" in c), (it, which, vocab, text, err)
+        if err is not None:
             raised += 1
             assert not getattr(o, "merges", None) or o.merges == {}, "a failed train() must not leave merges behind"
             continue
-        assert list(o.merges.items()) == list(r.merges.items()), (it, which, vocab, text)
-        assert o.vocab == r.vocab
+        assert list(o.merges.items()) == [((a, b), 256 + i) for i, (a, b) in enumerate(c["merges"])], (it, which, vocab, text)
+        want_vocab = {i: bytes([i]) for i in range(256)}
+        want_vocab.update({256 + i: bytes.fromhex(h) for i, h in enumerate(c["vocab_hex"])})
+        assert o.vocab == want_vocab
         probe = text[: 300] + " ab aab" + text[-50:]
-        assert o.encode(probe) == r.encode(probe), (it, which, probe)
-        assert o.decode(o.encode(probe)) == probe
-        r.save(os.path.join(tmp, "r")); o.save(os.path.join(tmp, "o"))
-        for ext in (".model", ".vocab"):
-            assert open(os.path.join(tmp, "r" + ext), "rb").read() == open(os.path.join(tmp, "o" + ext), "rb").read(), (it, ext)
+        ids = o.encode(probe)
+        assert (len(ids), sha(np.asarray(ids, dtype="<i4").tobytes())) == (c["probe_n_ids"], c["probe_ids_sha256"]), (it, which, probe)
+        assert o.decode(ids) == probe
+        o.save(os.path.join(tmp, "o"))
+        for ext in ("model", "vocab"):
+            assert sha(open(os.path.join(tmp, "o." + ext), "rb").read()) == c[ext + "_sha256"], (it, ext)
         done += 1
-    print(f"emu fuzz train ok: {done} trained identically, {raised} ran out of pairs on both sides, of {rounds}")
+    print(f"emu fuzz train ok: {done} trained identically, {raised} ran out of pairs on both sides, of {len(cases)}")
     return 0
 
 
 if __name__ == "__main__":
-    sys.exit(main(int(sys.argv[1]) if len(sys.argv) > 1 else 150, int(sys.argv[2]) if len(sys.argv) > 2 else 1))
+    sys.exit(main())

@@ -19,6 +19,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -51,8 +52,11 @@ def _pytest(lib, files, k=None, order=None, par=None):
     return subprocess.Popen(cmd, cwd=ROOT, env=env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
 
 
+DUMPS = {}      # --dump-outputs directories of the two bench jobs
+
+
 @pytest.fixture(scope="module")
-def jobs():
+def jobs(tmp_path_factory):
     sys.path.insert(0, EMU)
     import build_emu
     lib = build_emu.build()
@@ -76,19 +80,23 @@ def jobs():
                                       stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
     procs["fuzz"] = subprocess.Popen([sys.executable, os.path.join(EMU, "emu_fuzz_encode.py"), "120", "7"], cwd=ROOT, env=dict(_env(lib), EMU_PAR="3"),
                                      stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
-    # special-token front end (device) against the unmodified reference class (oracle/_ref, vendored by __graft_entry__.build())
-    procs["fuzz_special"] = subprocess.Popen([sys.executable, os.path.join(EMU, "emu_fuzz_special.py"), "100", "5"], cwd=ROOT, env=_env(lib),
+    # special-token front end (device) against the unmodified reference class (its answers: tests/golden/golden_fuzz_special.json)
+    procs["fuzz_special"] = subprocess.Popen([sys.executable, os.path.join(EMU, "emu_fuzz_special.py")], cwd=ROOT, env=_env(lib),
                                              stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
     # train() / encode() / save() of the classes against the unmodified reference classes on random small texts
-    procs["fuzz_train"] = subprocess.Popen([sys.executable, os.path.join(EMU, "emu_fuzz_train_ref.py"), "100", "5"], cwd=ROOT, env=_env(lib),
+    # (their answers: tests/golden/golden_fuzz_train.json)
+    procs["fuzz_train"] = subprocess.Popen([sys.executable, os.path.join(EMU, "emu_fuzz_train_ref.py")], cwd=ROOT, env=_env(lib),
                                            stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
     bench_args = ["--size-mib", "1", "--steps", "6", "--warmup", "3", "--strong-mib", "2", "--strong-sparse-at", "24", "--strong-check", "16",
                   "--encode-gb", "0.002", "--encode-merges", "200", "--encode-train-mib", "1", "--leg-budget-s", "600"]
     benv = dict(_env(lib), BPE_BENCH_EMU="1")
-    procs["bench1"] = subprocess.Popen([sys.executable, "bench.py", "--full-merges", "40"] + bench_args, cwd=ROOT, env=benv,
+    dump = tmp_path_factory.mktemp("bench_outputs")
+    DUMPS.update(bench1=str(dump / "one"), bench2=str(dump / "two"))
+    procs["bench1"] = subprocess.Popen([sys.executable, "bench.py", "--full-merges", "40", "--dump-outputs", DUMPS["bench1"]] + bench_args, cwd=ROOT, env=benv,
                                        stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True)
     procs["bench2"] = subprocess.Popen([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2",
-                                        "--master-addr", "127.0.0.1", "--master-port", str(_free_port()), "bench.py", "--gpus", "2"] + bench_args,
+                                        "--master-addr", "127.0.0.1", "--master-port", str(_free_port()), "bench.py", "--gpus", "2",
+                                        "--dump-outputs", DUMPS["bench2"]] + bench_args,
                                        cwd=ROOT, env=benv, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True)
     yield procs
     for p in procs.values():
@@ -143,19 +151,11 @@ def test_emu_encode_fuzz_under_guard_pages(jobs):
 
 
 def test_emu_special_tokens_fuzz_against_the_reference_class(jobs):
-    p = jobs["fuzz_special"]
-    out, _ = p.communicate(timeout=1500)
-    if p.returncode == 2:
-        pytest.skip("oracle/_ref is not vendored in this checkout (needs /root/reference once: __graft_entry__.build())")
-    assert p.returncode == 0 and "emu fuzz special ok" in out, out[-4000:]
+    assert "emu fuzz special ok" in _finish(jobs, "fuzz_special")
 
 
 def test_emu_train_fuzz_against_the_reference_classes(jobs):
-    p = jobs["fuzz_train"]
-    out, _ = p.communicate(timeout=1500)
-    if p.returncode == 2:
-        pytest.skip("oracle/_ref is not vendored in this checkout (needs /root/reference once: __graft_entry__.build())")
-    assert p.returncode == 0 and "emu fuzz train ok" in out, out[-4000:]
+    assert "emu fuzz train ok" in _finish(jobs, "fuzz_train")
 
 
 def _bench_line(jobs, name):
@@ -169,7 +169,12 @@ def _bench_line(jobs, name):
     assert p.returncode == 0, err[-6000:]
     lines = [ln for ln in out.splitlines() if ln.startswith("{")]
     assert len(lines) == 1, out[-2000:]          # the contract: ONE JSON line
-    return json.loads(lines[0])
+    d = json.loads(lines[0])
+    # --dump-outputs: the merges and counts of the K timed steps, float64
+    m, c = (np.load(os.path.join(DUMPS[name], f + ".npy")) for f in ("merges", "counts"))
+    assert m.dtype == c.dtype == np.float64 and m.shape == (d["steps"], 2) and c.shape == (d["steps"],)
+    assert m[:4].astype(int).tolist() == d["first_pairs"] and (c > 0).all()
+    return d
 
 
 CONTRACT_KEYS = ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline",

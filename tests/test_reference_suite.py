@@ -1,28 +1,22 @@
-"""CPU (this container only): the REFERENCE'S OWN test file, unmodified and in place (/root/reference/tests/test_tokenizer.py),
-run against minbpe_b200 through a two-line `minbpe` shim package — the drop-in claim, literally.  No GPU here, so the
-library under the classes is the CPU SIMT emulator build of the kernel sources (tests/emu/).  The 9 GPT4Tokenizer tests of
-that file need tiktoken's cl100k_base (a download) and are deselected.  Skipped where /root/reference does not exist."""
+"""CPU: the checks of the reference's own test file (karpathy/minbpe tests/test_tokenizer.py) against minbpe_b200 — the
+drop-in claim — with the reference's answers stored under tests/golden/ (golden_ref_suite.json), so that every result is
+also compared with the unmodified reference.  No GPU here, so the library under the classes is the CPU SIMT emulator build
+of the kernel sources (tests/emu/).  The 9 GPT4Tokenizer tests of that file need tiktoken's cl100k_base (a download) and
+are not part of it; 12 checks remain."""
 import os
 import subprocess
 import sys
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_TESTS = "/root/reference/tests/test_tokenizer.py"
 
 
-@pytest.mark.skipif(not os.path.exists(REF_TESTS), reason="the reference checkout is only present in the build container")
-def test_reference_test_file_passes_against_minbpe_b200(tmp_path):
+def test_reference_test_file_passes_against_minbpe_b200():
     sys.path.insert(0, os.path.join(ROOT, "tests", "emu"))
     import build_emu
     lib = build_emu.build()
-    shim = tmp_path / "minbpe"
-    shim.mkdir()
-    (shim / "__init__.py").write_text("from minbpe_b200 import *  # noqa\nfrom minbpe_b200 import BasicTokenizer, RegexTokenizer, GPT4Tokenizer, Tokenizer  # noqa\n")
-    env = dict(os.environ, BPE_LIB_PATH=lib, PYTHONPATH=f"{tmp_path}:{ROOT}", PYTHONDONTWRITEBYTECODE="1")
+    env = dict(os.environ, BPE_LIB_PATH=lib, PYTHONDONTWRITEBYTECODE="1")
     env.pop("PYTEST_CURRENT_TEST", None)
-    r = subprocess.run([sys.executable, "-m", "pytest", REF_TESTS, "-q", "-p", "no:cacheprovider", "-k", "not gpt4"],
-                       cwd=str(tmp_path), env=env, capture_output=True, text=True, timeout=900)
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "emu", "emu_reference_suite.py")],
+                       cwd=ROOT, env=env, capture_output=True, text=True, timeout=900)
     assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
-    assert "12 passed" in r.stdout, r.stdout[-1000:]
+    assert "reference suite ok: 12 passed" in r.stdout, r.stdout[-1000:]
