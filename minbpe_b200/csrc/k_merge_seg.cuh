@@ -5,8 +5,8 @@
 //
 //   read   4 * count bytes per segment        (one 1-D bulk async copy, TMA / UBLKCP, into the
 //                                              warp's private mbarrier ring, MS_STAGES deep)
-//   write  only from the first 128-token row that changed to the new end of the segment
-//          (16-byte stores, same address range); nothing for an untouched segment
+//   write  only from the 32-byte sector that holds the first changed word to the new end of the
+//          segment (16-byte stores, same address range); nothing for an untouched segment
 //   + 32-byte edge records per segment (first 3 / last 2 tokens, count), double-buffered, so a
 //     warp can see across its segment boundaries without reading a body that another warp rewrites
 //
@@ -85,34 +85,28 @@ struct SegArgs {
     u64 xstride;                  // the one of the current round's parity inside it, and `delta` is ignored
 };
 
-// one row (128 tokens, 4 per lane): merge starts m, kept tokens, replaced tokens written back to t[]
+// one row (128 tokens, 4 per lane) into bits 4R..4R+3 of the lane's masks: m = merge starts (a at the token, b after it),
+// pm = token 0 of the row follows an a (it is dropped if it is b).  Bits of tokens past the end of the segment are cleared
+// by the valid mask.
 template <int R>
-__device__ __forceinline__ void mark_row(u32 la, u32 lane, u32 count, u32 a, u32 b, u32 z, u32 (&t)[4], u32 &mn, u32 &keep,
-                                         u32 &dirty) {
+__device__ __forceinline__ void mark_row(u32 la, u32 a, u32 b, u32 (&t)[4], u32 &m, u32 &pm) {
     const uint4 q = lds128o<R * 512>(la);
     const u32 nx = lds32o<R * 512 + 16>(la), pv = lds32o<R * 512 - 4>(la);
     t[0] = q.x; t[1] = q.y; t[2] = q.z; t[3] = q.w;
-    u32 m = 0;
-    m |= (((t[0] ^ a) & TOK_MASK) == 0 && t[1] == b) ? 1u : 0u;
-    m |= (((t[1] ^ a) & TOK_MASK) == 0 && t[2] == b) ? 2u : 0u;
-    m |= (((t[2] ^ a) & TOK_MASK) == 0 && t[3] == b) ? 4u : 0u;
-    m |= (((t[3] ^ a) & TOK_MASK) == 0 && nx == b) ? 8u : 0u;
-    const u32 pm = (((pv ^ a) & TOK_MASK) == 0 && t[0] == b) ? 1u : 0u;
-    const u32 d = ((m << 1) | pm) & 0xfu;   // dropped: the token after a merge start
-    u32 valid = 0xfu;
-    if (R * 128u + 128u > count) {          // warp-uniform: the row that holds the end of the segment
-        const int rem = (int)count - (int)(R * 128 + lane * 4);
-        valid = rem >= 4 ? 0xfu : (rem <= 0 ? 0u : ((1u << rem) - 1u));
-    }
-    mn = m & valid;                         // a merge only starts at a token this segment owns
-    keep = ~d & valid;
-    dirty |= (mn | (keep ^ valid)) ? (1u << R) : 0u;
-    if (mn) {                               // few lanes: the merged token takes its place in the registers
-        if (mn & 1u) t[0] = z | (t[0] & TOK_FLAG);
-        if (mn & 2u) t[1] = z | (t[1] & TOK_FLAG);
-        if (mn & 4u) t[2] = z | (t[2] & TOK_FLAG);
-        if (mn & 8u) t[3] = z | (t[3] & TOK_FLAG);
-    }
+    m |= (((t[0] ^ a) & TOK_MASK) == 0 && t[1] == b) ? (1u << (4 * R)) : 0u;
+    m |= (((t[1] ^ a) & TOK_MASK) == 0 && t[2] == b) ? (2u << (4 * R)) : 0u;
+    m |= (((t[2] ^ a) & TOK_MASK) == 0 && t[3] == b) ? (4u << (4 * R)) : 0u;
+    m |= (((t[3] ^ a) & TOK_MASK) == 0 && nx == b) ? (8u << (4 * R)) : 0u;
+    pm |= (((pv ^ a) & TOK_MASK) == 0 && t[0] == b) ? (1u << (4 * R)) : 0u;
+}
+
+// the merged token takes the place of the merge start (bit 4R+i of mn) in the registers
+template <int R>
+__device__ __forceinline__ void replace_row(u32 mn, u32 z, u32 (&t)[4]) {
+    if (mn & (1u << (4 * R))) t[0] = z | (t[0] & TOK_FLAG);
+    if (mn & (2u << (4 * R))) t[1] = z | (t[1] & TOK_FLAG);
+    if (mn & (4u << (4 * R))) t[2] = z | (t[2] & TOK_FLAG);
+    if (mn & (8u << (4 * R))) t[3] = z | (t[3] & TOK_FLAG);
 }
 
 // write the kept tokens of one row to their compacted place (word offset `off` of the stage)
@@ -271,16 +265,24 @@ __global__ void __launch_bounds__(MS_THREADS, MS_MINBLOCKS) k_merge_seg(SegArgs 
         if (lane < 3) sts32(s_a + (count + lane) * 4, lds32(meta_a + 8 + lane * 4));   // the three tokens that follow
         __syncwarp();
 
-        // ---- mark: row r = tokens [128r, 128r+128), four consecutive tokens per lane ----
-        u32 t[4][4], mn[4] = {0, 0, 0, 0}, keep[4] = {0, 0, 0, 0};
-        u32 dirty = 0;
+        // ---- mark: row r = tokens [128r, 128r+128), four consecutive tokens per lane.  A lane's 16 tokens are bits
+        //      4r+i of its masks; in that order their stream positions 128r + 4*lane + i increase, so the tokens this
+        //      segment owns (position < count) are a prefix of the bits ----
+        u32 t[4][4], m = 0, pm = 0;
         const u32 la = s_a + lane * 16;
-        mark_row<0>(la, lane, count, a, b, z, t[0], mn[0], keep[0], dirty);
-        if (count > 128u) mark_row<1>(la, lane, count, a, b, z, t[1], mn[1], keep[1], dirty);
-        if (count > 256u) mark_row<2>(la, lane, count, a, b, z, t[2], mn[2], keep[2], dirty);
-        if (count > 384u) mark_row<3>(la, lane, count, a, b, z, t[3], mn[3], keep[3], dirty);
-        dirty = __reduce_or_sync(FULL, dirty);   // rows in which some token is replaced or dropped
-        if (!dirty) {
+        mark_row<0>(la, a, b, t[0], m, pm);
+        if (count > 128u) mark_row<1>(la, a, b, t[1], m, pm);   // short segments (the sparse end of training) skip rows
+        if (count > 256u) mark_row<2>(la, a, b, t[2], m, pm);
+        if (count > 384u) mark_row<3>(la, a, b, t[3], m, pm);
+        const u32 nvalid = 4u * (count >> 7) + (u32)min(max((int)(count & 127u) - (int)(4u * lane), 0), 4);
+        const u32 valid = (1u << nvalid) - 1u;
+        const u32 mn = m & valid;                                  // a merge only starts at a token this segment owns
+        const u32 keep = ~(((m << 1) & 0xeeeeu) | pm) & valid;     // dropped: the token after a merge start
+        // lowest position whose word changes (a merge start or a dropped token); rows and words in front of it stay
+        const u32 ch = mn | (keep ^ valid);
+        const u32 cb = __ffs(ch) - 1u;
+        const u32 first = ~__reduce_max_sync(FULL, ch ? ~((cb >> 2) * 128u + lane * 4u + (cb & 3u)) : 0u);   // MS_INVALID: none
+        if (first == MS_INVALID) {
             // untouched segment: nothing to write, the edge record carries over
             if (lane < 8) reinterpret_cast<u32 *>(&e_next[seg])[lane] = lds32(meta_a + 32 + lane * 4);
             __syncwarp();
@@ -289,7 +291,7 @@ __global__ void __launch_bounds__(MS_THREADS, MS_MINBLOCKS) k_merge_seg(SegArgs 
 
         // ---- statistics delta of this segment's merge starts (reads the stage before it is rewritten) ----
         if (delta) {
-            u32 mall = mn[0] | (mn[1] << 4) | (mn[2] << 8) | (mn[3] << 12);
+            u32 mall = mn;
 #pragma unroll 1
             while (mall) {   // one pass per merge start of this lane
                 const int bit = __ffs(mall) - 1;
@@ -298,8 +300,15 @@ __global__ void __launch_bounds__(MS_THREADS, MS_MINBLOCKS) k_merge_seg(SegArgs 
             }
         }
 
+        if (mn) {   // few lanes
+            replace_row<0>(mn, z, t[0]);
+            replace_row<1>(mn, z, t[1]);
+            replace_row<2>(mn, z, t[2]);
+            replace_row<3>(mn, z, t[3]);
+        }
+
         // ---- kept tokens per lane and row, packed one byte per row: one warp scan for all four rows ----
-        const u32 own = __popc(keep[0]) | (__popc(keep[1]) << 8) | (__popc(keep[2]) << 16) | (__popc(keep[3]) << 24);
+        const u32 own = __popc(keep & 0xfu) | (__popc(keep & 0xf0u) << 8) | (__popc(keep & 0xf00u) << 16) | (__popc(keep & 0xf000u) << 24);
         u32 incl = own;
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) {
@@ -311,24 +320,24 @@ __global__ void __launch_bounds__(MS_THREADS, MS_MINBLOCKS) k_merge_seg(SegArgs 
         const u32 k0 = tot & 0xffu, k1 = (tot >> 8) & 0xffu, k2 = (tot >> 16) & 0xffu, k3 = tot >> 24;
         const u32 off1 = k0, off2 = k0 + k1, off3 = off2 + k2;
         const u32 new_count = off3 + k3;
-        const int first_dirty = __ffs(dirty) - 1;   // rows in front of it stay where they are
+        const u32 first_row = first >> 7;           // rows in front of it stay where they are
         __syncwarp();                               // all lanes hold their tokens; delta reads are done
 
-        // ---- compact in place inside the stage, from the first dirty row on ----
-        if (first_dirty <= 0) scatter_row(s_a, lane, 0u, k0, excl & 0xffu, keep[0], t[0]);
-        if (first_dirty <= 1 && count > 128u) scatter_row(s_a, lane, off1, k1, (excl >> 8) & 0xffu, keep[1], t[1]);
-        if (first_dirty <= 2 && count > 256u) scatter_row(s_a, lane, off2, k2, (excl >> 16) & 0xffu, keep[2], t[2]);
-        if (count > 384u) scatter_row(s_a, lane, off3, k3, excl >> 24, keep[3], t[3]);
+        // ---- compact in place inside the stage, from the first changed row on (a row past the end keeps nothing) ----
+        if (first_row == 0) scatter_row(s_a, lane, 0u, k0, excl & 0xffu, keep & 0xfu, t[0]);
+        if (first_row <= 1 && k1) scatter_row(s_a, lane, off1, k1, (excl >> 8) & 0xffu, (keep >> 4) & 0xfu, t[1]);
+        if (first_row <= 2 && k2) scatter_row(s_a, lane, off2, k2, (excl >> 16) & 0xffu, (keep >> 8) & 0xfu, t[2]);
+        if (k3) scatter_row(s_a, lane, off3, k3, excl >> 24, keep >> 12, t[3]);
         __syncwarp();
-        // ---- copy-out: 16-byte vectors from the first dirty row to the new end (the up to three
-        //      words past new_count land in the dead part of the segment) ----
+        // ---- copy-out: 16-byte vectors from the 32-byte sector that holds the first changed word to the new end (the
+        //      up to three words past new_count land in the dead part of the segment) ----
         {
             uint4 *__restrict__ gp = reinterpret_cast<uint4 *>(w + (u64)seg * SEG_TOKENS) + lane;
-            const u32 vend = (new_count + 3u) >> 2;
-            if (first_dirty <= 0 && lane < vend) gp[0] = lds128o<0>(la);
-            if (first_dirty <= 1 && lane + 32u < vend) gp[32] = lds128o<512>(la);
-            if (first_dirty <= 2 && lane + 64u < vend) gp[64] = lds128o<1024>(la);
-            if (lane + 96u < vend) gp[96] = lds128o<1536>(la);
+            const u32 vend = (new_count + 3u) >> 2, vbeg = (first >> 3) * 2u;
+            if (lane >= vbeg && lane < vend) gp[0] = lds128o<0>(la);
+            if (lane + 32u >= vbeg && lane + 32u < vend) gp[32] = lds128o<512>(la);
+            if (lane + 64u >= vbeg && lane + 64u < vend) gp[64] = lds128o<1024>(la);
+            if (lane + 96u >= vbeg && lane + 96u < vend) gp[96] = lds128o<1536>(la);
         }
         // ---- the segment's new edge record ----
         {
