@@ -141,6 +141,16 @@ int bpe_encode_text_gpt4_special(bpe_handle *h, const uint8_t *bytes, uint64_t n
                                  const uint8_t *byte_perm, const uint8_t *special_bytes, const uint32_t *special_offsets,
                                  const int32_t *special_ids, int32_t n_special, int32_t *out_ids, uint64_t out_cap,
                                  uint64_t *out_n);
+/* [tok.encode(t, allowed_special) for t in docs] in one call (regex.py:123-164 per document).  bytes = the n_docs documents'
+ * UTF-8 joined by single 0xFF bytes (a byte UTF-8 never contains); every document is split (BPE_OPT_SPLIT_PATTERN) and
+ * special-token-cut on its own.  Specials as in bpe_encode_text_gpt4_special (n_special = 0: none).  out_doc_offsets[n_docs + 1]:
+ * document d's ids are out_ids[out_doc_offsets[d] .. out_doc_offsets[d + 1]).  BPE_ERR_ARG if bytes does not hold exactly
+ * n_docs - 1 separators. */
+int bpe_encode_batch_gpt4(bpe_handle *h, const uint8_t *bytes, uint64_t n, uint64_t n_docs,
+                          const int32_t *merges, int32_t n_merges, const uint8_t *byte_perm,
+                          const uint8_t *special_bytes, const uint32_t *special_offsets, const int32_t *special_ids,
+                          int32_t n_special, int32_t *out_ids, uint64_t out_cap, uint64_t *out_n,
+                          uint64_t *out_doc_offsets);
 /* Counters of the memoised encode: out[0] distinct chunks in the memo table, [1] ids in its pool; of the last call:
  * [2] chunks newly added, [3] chunks encoded directly (no room in the table, or longer than 48 bytes), [4] of which
  * long, [5] pieces, [6] pieces that took the general path, [7] device microseconds of the encode kernels

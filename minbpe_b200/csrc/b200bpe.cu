@@ -24,6 +24,7 @@
 #include "k_xchg.cuh"
 #include "k_encode2.cuh"
 #include "k_special.cuh"
+#include "k_batch.cuh"
 
 #define BPE_ABI_VERSION 1
 
@@ -947,4 +948,5 @@ extern "C" int bpe_debug_table(bpe_handle *h, int32_t *pairs, int64_t *counts, u
 #include "special_host.inl"
 #include "split_host.inl"
 #include "encode2_host.inl"
+#include "batch_host.inl"
 #include "decode_host.inl"

@@ -37,6 +37,7 @@
 #define E2_HALO 64                        // bytes after the tile that its chunks may reach into (>= E2_LMAX + 4, multiple of 32)
 #define E2_OUT (E2_TILE + E2_LMAX)           // ids of one tile staged in shared memory by k_enc_write
 #define E2_PENDING 0xffu                  // MemoSlot.ntok while the slot has not been encoded yet
+#define BATCH_SEP 0xffu                   // document separator of the batched encode (k_batch.cuh): a byte UTF-8 never contains
 
 struct __align__(16) MemoSlot {           // 64 bytes
     u64 tag;                              // 0 = empty, else (hash | 1)
@@ -171,6 +172,8 @@ __device__ __forceinline__ void e2_direct_append(const Enc2 &E, u64 pos, bool is
 }
 
 // ---- pass 1: claim memo slots ------------------------------------------------------------------------------
+// BATCH (k_batch.cuh): a chunk whose first byte is 0xFF is a document separator — never memoised, no ids, never a failure
+template <bool BATCH>
 __global__ void __launch_bounds__(E2_THREADS) k_enc_insert(Enc2 E) {
     __shared__ __align__(16) unsigned char s_b[E2_TILE + E2_HALO + 8];
     __shared__ u32 s_bits[(E2_TILE + E2_HALO) / 32 + 2];
@@ -185,6 +188,7 @@ __global__ void __launch_bounds__(E2_THREADS) k_enc_insert(Enc2 E) {
         mine &= mine - 1;
         const u32 p = base + k;
         if (lo + p >= E.n) break;
+        if (BATCH && s_b[p] == BATCH_SEP) continue;
         const u32 len = e2_chunk_len(T, p);
         if (len > E2_LMAX) { e2_direct_append(E, lo + p, true); continue; }
         u32 kw[E2_KW];
@@ -463,41 +467,60 @@ __device__ __forceinline__ bool e2_resolve(const Enc2 &E, const E2Tile &T, u64 l
 }
 
 // ---- pass 4: ids per tile -------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(E2_THREADS) k_enc_count(Enc2 E, u32 *__restrict__ part) {
+// BATCH: also the number of separators of the tile -> sep_part
+template <bool BATCH>
+__global__ void __launch_bounds__(E2_THREADS) k_enc_count(Enc2 E, u32 *__restrict__ part, u32 *__restrict__ sep_part) {
     __shared__ __align__(16) unsigned char s_b[E2_TILE + E2_HALO + 8];
     __shared__ u32 s_bits[(E2_TILE + E2_HALO) / 32 + 2];
     __shared__ u32 s_red[E2_THREADS / 32];
+    __shared__ u32 s_red_sep[BATCH ? E2_THREADS / 32 : 1];
     const E2Tile T{s_b, s_bits};
     const u64 lo = (u64)blockIdx.x * E2_TILE;
     if (threadIdx.x < 2) s_bits[(E2_TILE + E2_HALO) / 32 + threadIdx.x] = 0xffffffffu;
     e2_load_tile(E, lo, T);
     const u32 base = threadIdx.x * E2_ITEMS;
     u32 mine = (s_bits[base >> 5] >> (base & 31u)) & 0xffu;
-    u32 sum = 0;
+    u32 sum = 0, nsep = 0;
     while (mine) {
         const u32 k = __ffs(mine) - 1;
         mine &= mine - 1;
         const u32 p = base + k;
         if (lo + p >= E.n) break;
+        if (BATCH && s_b[p] == BATCH_SEP) { ++nsep; continue; }
         u32 nt = 0, off = 0;
         if (e2_resolve(E, T, lo, p, nt, off)) sum += nt; else atomicOr(&E.ctl->fail, E2_FAIL_OTHER);
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
     if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = sum;
+    if (BATCH) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) nsep += __shfl_xor_sync(0xffffffffu, nsep, o);
+        if ((threadIdx.x & 31) == 0) s_red_sep[threadIdx.x >> 5] = nsep;
+    }
     __syncthreads();
     if (threadIdx.x == 0) {
         u32 t = 0;
         for (int w = 0; w < E2_THREADS / 32; ++w) t += s_red[w];
         part[blockIdx.x] = t;
+        if (BATCH) {
+            u32 c = 0;
+            for (int w = 0; w < E2_THREADS / 32; ++w) c += s_red_sep[w];
+            sep_part[blockIdx.x] = c;
+        }
     }
 }
 
 // ---- pass 5: write the ids ------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(E2_THREADS) k_enc_write(Enc2 E, const u64 *__restrict__ excl, int *__restrict__ out) {
+// BATCH: separator s of the piece (sep_excl[tile] + the separators in front of it in the tile) closes a document:
+// doc_out[s] = out_base + its output position
+template <bool BATCH>
+__global__ void __launch_bounds__(E2_THREADS) k_enc_write(Enc2 E, const u64 *__restrict__ excl, int *__restrict__ out,
+                                                          const u64 *__restrict__ sep_excl, u64 *__restrict__ doc_out, u64 out_base) {
     __shared__ __align__(16) unsigned char s_b[E2_TILE + E2_HALO + 8];
     __shared__ u32 s_bits[(E2_TILE + E2_HALO) / 32 + 2];
     __shared__ u32 s_scan[E2_THREADS / 32];
+    __shared__ u32 s_scan_sep[BATCH ? E2_THREADS / 32 : 1];
     // ids of the tile's chunks in output order: the first E2_OUT of them are staged here and stored coalesced; a
     // long chunk that starts in this tile can carry more ids than the tile has bytes — those go straight to HBM
     __shared__ u32 s_out[E2_OUT];
@@ -511,11 +534,13 @@ __global__ void __launch_bounds__(E2_THREADS) k_enc_write(Enc2 E, const u64 *__r
     u32 nts[E2_ITEMS], offs[E2_ITEMS];
     u32 sum = 0, cnt = 0;
     u32 mine = bits;
+    u32 sep_bits = 0, nsep = 0;     // BATCH: bit c = chunk c of this thread is a separator
     while (mine) {
         const u32 k = __ffs(mine) - 1;
         mine &= mine - 1;
         const u32 p = base + k;
         if (lo + p >= E.n) break;
+        if (BATCH && s_b[p] == BATCH_SEP) { sep_bits |= 1u << cnt; ++nsep; nts[cnt] = 0; offs[cnt] = 0; ++cnt; continue; }
         u32 nt = 0, off = 0;
         e2_resolve(E, T, lo, p, nt, off);
         nts[cnt] = nt; offs[cnt] = off; ++cnt;
@@ -525,12 +550,29 @@ __global__ void __launch_bounds__(E2_THREADS) k_enc_write(Enc2 E, const u64 *__r
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) { const u32 v = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= (u32)o) incl += v; }
     if (lane == 31) s_scan[warp] = incl;
+    u32 sep_incl = 0;
+    if constexpr (BATCH) {
+        sep_incl = nsep;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) { const u32 v = __shfl_up_sync(0xffffffffu, sep_incl, o); if (lane >= (u32)o) sep_incl += v; }
+        if (lane == 31) s_scan_sep[warp] = sep_incl;
+    }
     __syncthreads();
     u32 wbase = 0, total = 0;
 #pragma unroll
     for (int w = 0; w < E2_THREADS / 32; ++w) { const u32 v = s_scan[w]; if ((u32)w < warp) wbase += v; total += v; }
     u32 dst = wbase + incl - sum;
     int *o = out + excl[blockIdx.x];
+    if constexpr (BATCH) if (sep_bits) {
+        u64 s = sep_excl[blockIdx.x] + sep_incl - nsep;
+#pragma unroll
+        for (int w = 0; w < E2_THREADS / 32; ++w) if ((u32)w < warp) s += s_scan_sep[w];
+        u32 d = dst;
+        for (u32 c = 0; c < cnt; ++c) {
+            if ((sep_bits >> c) & 1u) doc_out[s++] = out_base + excl[blockIdx.x] + d;
+            d += nts[c];
+        }
+    }
     for (u32 c = 0; c < cnt; ++c) {
         const u32 nt = nts[c], off = offs[c];
         for (u32 j = 0; j < nt; ++j) {

@@ -60,6 +60,7 @@ def load_library():
         "bpe_encode": ([vp, vp, u64, vp, u64, vp, i32, vp, vp, u64, P(u64)], ci),
         "bpe_encode_text_gpt4": ([vp, vp, u64, vp, i32, vp, vp, u64, P(u64)], ci),
         "bpe_encode_text_gpt4_special": ([vp, vp, u64, vp, i32, vp, vp, vp, vp, i32, vp, u64, P(u64)], ci),
+        "bpe_encode_batch_gpt4": ([vp, vp, u64, u64, vp, i32, vp, vp, vp, vp, i32, vp, u64, P(u64), vp], ci),
         "bpe_encode_stats": ([vp, vp], ci),
         "bpe_get_timing": ([vp, P(Timing)], ci),
         "bpe_set_option": ([vp, ci, i64], ci),
@@ -250,6 +251,29 @@ class Engine:
         self._check(self._lib.bpe_encode_text_gpt4(self._h, _ptr(b) if b.size else None, b.size, _ptr(m) if m.size else None,
                                                    m.shape[0], _ptr(perm), _ptr(out), out.size, ctypes.byref(n)), "bpe_encode_text_gpt4")
         return out[: n.value]
+
+    def encode_batch_gpt4(self, data, n_docs, merges, byte_perm=None, specials=None):
+        """-> (ids int32, doc_offsets int64[n_docs + 1]): the n_docs documents of `data` (their utf-8 joined by single 0xFF
+        bytes) each split (BPE_OPT_SPLIT_PATTERN), special-token-cut and encoded on its own, all in one call; document d is
+        ids[doc_offsets[d]:doc_offsets[d + 1]].  specials as in encode_text_gpt4."""
+        self._ensure_gpt4_tables()
+        b = np.frombuffer(data, dtype=np.uint8) if not isinstance(data, np.ndarray) else np.ascontiguousarray(data, dtype=np.uint8)
+        m = np.ascontiguousarray(np.asarray(merges, dtype=np.int32).reshape(-1, 2))
+        perm = None if byte_perm is None else np.ascontiguousarray(byte_perm, dtype=np.uint8)
+        out = np.empty(max(b.size, 1), dtype=np.int32)          # every id covers at least one byte; separators give none
+        doc = np.zeros(int(n_docs) + 1, dtype=np.uint64)
+        blob, offs, ids, k = None, None, None, 0
+        if specials:
+            blob = np.frombuffer(b"".join(t for t, _ in specials), dtype=np.uint8)
+            offs = np.zeros(len(specials) + 1, dtype=np.uint32)
+            np.cumsum([len(t) for t, _ in specials], out=offs[1:])
+            ids = np.asarray([i for _, i in specials], dtype=np.int32)
+            k = len(specials)
+        n = ctypes.c_uint64()
+        self._check(self._lib.bpe_encode_batch_gpt4(
+            self._h, _ptr(b) if b.size else None, b.size, int(n_docs), _ptr(m) if m.size else None, m.shape[0], _ptr(perm),
+            _ptr(blob), _ptr(offs), _ptr(ids), k, _ptr(out), out.size, ctypes.byref(n), _ptr(doc)), "bpe_encode_batch_gpt4")
+        return out[: n.value], doc.astype(np.int64)
 
     def encode_stats(self):
         a = np.zeros(10, dtype=np.uint64)

@@ -81,6 +81,16 @@ def render_token(t: bytes) -> str:
     return replace_control_characters(t.decode("utf-8", errors="replace"))
 
 
+def _batch_result(lists, flat):
+    """encode_batch's two forms from per-document id lists: the lists, or (ids int32, offsets int64[len + 1])."""
+    if not flat:
+        return lists
+    offsets = np.zeros(len(lists) + 1, dtype=np.int64)
+    np.cumsum([len(x) for x in lists], out=offsets[1:])
+    ids = np.fromiter((i for x in lists for i in x), dtype=np.int32, count=int(offsets[-1]))
+    return ids, offsets
+
+
 def _vocab_from_merges(merges, special_tokens):
     """base.py:88-95: 256 byte tokens, then merges in order, then specials."""
     vocab = {i: bytes((i,)) for i in range(256)}
@@ -183,6 +193,11 @@ class Tokenizer:
 
     def decode(self, ids):
         raise NotImplementedError
+
+    def encode_batch(self, texts, *, flat=False):
+        """[self.encode(t) for t in texts] (not in the reference).  flat=True: (ids int32, offsets int64 of len(texts) + 1)
+        instead, document i being ids[offsets[i]:offsets[i + 1]]."""
+        return _batch_result([self.encode(t) for t in texts], flat)
 
     def _build_vocab(self):
         return _vocab_from_merges(self.merges, self.special_tokens)
@@ -426,19 +441,58 @@ class RegexTokenizer(Tokenizer):
             return []
         return self.engine.encode(data, offsets, self._merge_array(), self._byte_perm).tolist()
 
+    def encode_ordinary_batch(self, texts, *, flat=False):
+        """[self.encode_ordinary(t) for t in texts] (not in the reference); flat as in encode_batch.  Batches of at least
+        DEVICE_SPLIT_MIN_BYTES under the GPT-2 / GPT-4 pattern are split and encoded in one device call."""
+        return self._encode_batch(texts, None, flat)
+
+    def encode_batch(self, texts, allowed_special="none_raise", *, flat=False):
+        """[self.encode(t, allowed_special) for t in texts] (not in the reference): same ids, same errors.  flat=True:
+        (ids int32, offsets int64 of len(texts) + 1), document i being ids[offsets[i]:offsets[i + 1]] — no Python list per
+        id.  Batches of at least DEVICE_SPLIT_MIN_BYTES under the GPT-2 / GPT-4 pattern, with special tokens the device
+        front end takes, are split and encoded in one device call (bpe_encode_batch_gpt4); others loop over encode()."""
+        return self._encode_batch(texts, allowed_special, flat)
+
+    def _encode_batch(self, texts, allowed_special, flat):
+        texts = list(texts)
+        if not texts:
+            return _batch_result([], flat)
+        if allowed_special is None:
+            special, one = {}, self.encode_ordinary
+        else:
+            special = self._resolve_special(allowed_special)
+            one = lambda t: self.encode(t, allowed_special)     # noqa: E731
+        if not self.merges or (special and not self._device_specials(special)):
+            return _batch_result([one(t) for t in texts], flat)
+        raws = []
+        for t in texts:      # encode()'s checks, document by document: the first failing document raises what the loop would
+            if allowed_special == "none_raise":
+                assert all(token not in t for token in self.special_tokens)
+            raws.append(t.encode("utf-8"))
+        if not self._device_split(sum(map(len, raws))):
+            return _batch_result([one(t) for t in texts], flat)
+        spec = [(k.encode("utf-8"), int(v)) for k, v in special.items()] or None
+        ids, offsets = self.engine.encode_batch_gpt4(b"\xff".join(raws), len(raws), self._merge_array(), self._byte_perm, specials=spec)
+        if flat:
+            return ids, offsets
+        flat_ids, o = ids.tolist(), offsets.tolist()
+        return [flat_ids[o[i]:o[i + 1]] for i in range(len(raws))]
+
+    def _resolve_special(self, allowed_special):
+        """regex.py:131-145: the specials allowed_special selects ("none_raise": none; the caller checks the text)."""
+        if allowed_special == "all":
+            return self.special_tokens
+        if allowed_special in ("none", "none_raise"):
+            return {}
+        if isinstance(allowed_special, set):
+            return {k: v for k, v in self.special_tokens.items() if k in allowed_special}
+        raise ValueError(f"allowed_special={allowed_special} not understood")
+
     def encode(self, text, allowed_special="none_raise"):
         """regex.py:123-164."""
-        if allowed_special == "all":
-            special = self.special_tokens
-        elif allowed_special == "none":
-            special = {}
-        elif allowed_special == "none_raise":
-            special = {}
+        special = self._resolve_special(allowed_special)
+        if allowed_special == "none_raise":
             assert all(token not in text for token in self.special_tokens)
-        elif isinstance(allowed_special, set):
-            special = {k: v for k, v in self.special_tokens.items() if k in allowed_special}
-        else:
-            raise ValueError(f"allowed_special={allowed_special} not understood")
         if not special:
             return self.encode_ordinary(text)
         if self.merges and self._device_specials(special):

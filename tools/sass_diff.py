@@ -37,7 +37,8 @@ def kernels(so):
 def main():
     old, new = kernels(sys.argv[1]), kernels(sys.argv[2])
     alias = {"k_merge_seg": "k_merge_seg<false>", "k_split_apply<false>": "k_split_apply<false,false,0>",
-             "k_split_apply<true>": "k_split_apply<true,false,0>", "k_split_reduce": "k_split_reduce<false>"}    # became templates
+             "k_split_apply<true>": "k_split_apply<true,false,0>", "k_split_reduce": "k_split_reduce<false>",
+             "k_enc_insert": "k_enc_insert<false>", "k_enc_count": "k_enc_count<false>", "k_enc_write": "k_enc_write<false>"}    # became templates
     same = diff = gone = 0
     for k in sorted(old):
         k2 = k if k in new else alias.get(k)
